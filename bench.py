@@ -13,15 +13,22 @@ collective; torch.distributed is used only for the barrier and the max-over-rank
          H2D of the samples and D2H of the PAF records inside the timed region
   --impl reference   the reference's own CPU mapper (oracle/_ref, else the oracle port) on
          all host cores over a bounded sample of the same workload
+
+The benchmark writes nothing into the source tree (which may be read-only): the synthetic index is
+built in a temporary directory that is removed at exit.
 """
 import argparse
+import atexit
 import json
 import os
+import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
+sys.dont_write_bytecode = True
 ROOT = os.path.dirname(os.path.abspath(__file__))
 for p in (ROOT, os.path.join(ROOT, "tests"), os.path.join(ROOT, "tools")):
     sys.path.insert(0, p)
@@ -33,12 +40,24 @@ GENOME = "g4m7"
 N_READS = 10000
 N_SAMPLES = 4000
 NOISE_MULT = 1.5          # SURVEY.md 8(d): noise N(0, 1.5 * level_stdv)
+DUMP_BYTES = 64 << 20     # --dump-outputs writes at most this much
+
+_data_dir = None
+
+
+def data_dir():
+    """Per-process scratch directory for the synthetic index, removed at exit."""
+    global _data_dir
+    if _data_dir is None:
+        _data_dir = tempfile.mkdtemp(prefix="uncalled_b200_bench_")
+        atexit.register(shutil.rmtree, _data_dir, True)
+    return _data_dir
 
 
 def workload(rank, n_reads=N_READS):
     import synth
     import synthdata
-    prefix, g = synthdata.get_index(GENOME)
+    prefix, g = synthdata.get_index(GENOME, data_dir())
     sig, truth = synth.reads(g, n_reads, N_SAMPLES, seed=7 + 1000 * rank, noise_mult=NOISE_MULT)
     return prefix, sig
 
@@ -290,7 +309,7 @@ def run_stream_workload(args, rank, local_rank, world):
     total_channels, chunk_len = 512, 450
     n_channels = (total_channels + world - 1 - rank) // world       # channel c lives on rank c % world
     n_reads = n_channels * args.reads_per_channel
-    prefix, g = synthdata.get_index(GENOME)
+    prefix, g = synthdata.get_index(GENOME, data_dir())
     sig, _ = synth.reads(g, n_reads, N_SAMPLES, seed=7 + 1000 * rank, noise_mult=NOISE_MULT)
     sigs = [sig[i] for i in range(n_reads)]
     idx = U.Index(prefix, device=local_rank)
@@ -373,7 +392,7 @@ def run_fast5_workload(args, rank, local_rank, world):
     path = os.path.join(ROOT, "bench_data", "bench_reads_4000x4000.fast5")
     if not os.path.exists(path):
         raise SystemExit("bench_data/bench_reads_4000x4000.fast5 is missing: run tools/make_bench_fast5.py where /root/reference exists")
-    prefix, _ = synthdata.get_index(GENOME)
+    prefix, _ = synthdata.get_index(GENOME, data_dir())
     cpus = host_cpus()
     threads = max(1, cpus["usable"] // world)
     my_files = [path for i in range(args.files) if i % world == rank]
@@ -447,6 +466,22 @@ def run_fast5_workload(args, rank, local_rank, world):
         dist.destroy_process_group()
 
 
+def dump_outputs(out_dir, recs):
+    """The PAF records a caller of the timed path receives, one DIR/paf_<field>.npy per field (float64 holds every
+    field exactly), and DIR/read_index.npy naming their reads: all of them, or a fixed seeded sample when all of them
+    would take more than DUMP_BYTES."""
+    fields = recs.dtype.names
+    per_read = 8 * (len(fields) + 1)
+    ids = np.arange(len(recs))
+    budget = (DUMP_BYTES - 128 * (len(fields) + 1)) // per_read        # 128 bytes: the header of a .npy file
+    if len(recs) > budget:
+        ids = np.sort(np.random.default_rng(0).choice(len(recs), budget, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "read_index.npy"), ids.astype(np.float64))
+    for f in fields:
+        np.save(os.path.join(out_dir, "paf_%s.npy" % f), recs[f][ids].astype(np.float64))
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -471,7 +506,12 @@ def main():
     ap.add_argument("--files", type=int, default=16, help="fast5 workload: total number of 4000-read files (all ranks together)")
     ap.add_argument("--batch-reads", type=int, default=8000, help="fast5 workload: reads per GPU batch")
     ap.add_argument("--reads-per-channel", type=int, default=2)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="batch workload: after the timed steps, write the PAF records of the last timed step (rank 0) to "
+                         "DIR as float64 .npy files, one per field, for comparing two builds on identical inputs")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "batch"):
+        ap.error("--dump-outputs is available for the batch workload of --impl ours only")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -499,11 +539,7 @@ def main():
         return
 
     n_reads = args.reads
-    if world > 1 and rank != 0:
-        dist.barrier()           # rank 0 builds the shared index cache first
     prefix, sig = workload(rank, n_reads)
-    if world > 1 and rank == 0:
-        dist.barrier()
     descs = U.make_descs([N_SAMPLES] * n_reads)
     idx = U.Index(prefix, device=local_rank)
     bm = U.BatchMapper(idx, max_reads=n_reads, max_samples=n_reads * N_SAMPLES)
@@ -617,6 +653,9 @@ def main():
         exact_ties = {"value": world * n_reads / (ex_ms / 1e3), "unit": "reads/s", "steps": 1, "ms_per_step": ex_ms,
                       "reads_with_a_PAF_field_differing_from_default_kernel": int(np.any([recs_e[k] != out_dev[k] for k in paf_fields], axis=0).sum()),
                       "note": "k2_map_exact, device-resident samples, CUDA events, max over ranks"}
+
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out_dev)
 
     ms_per_step = dev_ms / args.steps
     value = world * n_reads / (ms_per_step / 1e3)

@@ -15,6 +15,9 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 ORACLE_DIR = os.path.join(ROOT, "oracle")
 GOLDEN = os.path.join(ROOT, "tests", "golden")
 MODEL_TABLE = os.path.join(ROOT, "uncalled_b200", "data", "r94_5mer_template.f32")
+# what the reference's own code returns on the tests' seeded inputs (tools/make_reference_checks_golden.py)
+REFERENCE_CHECKS_JSON = os.path.join(GOLDEN, "reference_checks.json")
+REFERENCE_CHECKS_NPZ = os.path.join(GOLDEN, "reference_checks.npz")
 
 u8p = C.POINTER(C.c_uint8)
 f32p = C.POINTER(C.c_float)
@@ -69,10 +72,15 @@ def paf_tuple(r):
 
 
 def build_oracle():
-    """Compile the C restatement (and oracle/_ref when /root/reference is present)."""
+    """Compile the C restatement."""
     subprocess.run(["make", "-C", ORACLE_DIR, "libunc_oracle.so"], check=True, capture_output=True)
-    if os.path.isdir("/root/reference/src"):
-        subprocess.run(["make", "-C", ORACLE_DIR, "ref"], check=True, capture_output=True)
+
+
+def reference_checks(section):
+    """The stored records of one section of tests/golden/reference_checks.json."""
+    import json
+    with open(REFERENCE_CHECKS_JSON) as f:
+        return json.load(f)[section]
 
 
 _orc = None

@@ -12,12 +12,12 @@ import synth  # noqa: E402
 CACHE = os.path.join(ROOT, "bench_data")
 
 
-def get_index(name):
-    """Returns (prefix, genome array).  Builds into bench_data/ on first use."""
+def get_index(name, cache=CACHE):
+    """Returns (prefix, genome array).  Builds into `cache` (bench_data/ by default) on first use."""
     import ctypes as C
     meta = json.load(open(os.path.join(ROOT, "tests", "golden", "synth_uncl.json")))[name]
-    os.makedirs(CACHE, exist_ok=True)
-    prefix = os.path.join(CACHE, name)
+    os.makedirs(cache, exist_ok=True)
+    prefix = os.path.join(cache, name)
     g = synth.genome(meta["size"], meta["seed"])
     if not all(os.path.exists(prefix + e) for e in (".bwt", ".sa", ".ann", ".amb", ".pac", ".uncl")):
         fa = prefix + ".fa"

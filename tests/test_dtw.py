@@ -1,5 +1,5 @@
-"""DTW (SURVEY 8(f) rank 4; reference src/dtw.hpp): the oracle's restatement against the reference's own DTWr94p / DTWr94d
-(oracle/_ref, where built), the device routine under the emulator against the oracle, and -- on the GPU -- unc_dtw_batch
+"""DTW (SURVEY 8(f) rank 4; reference src/dtw.hpp): the oracle's restatement against what the reference's own DTWr94p / DTWr94d
+return (stored in tests/golden/reference_checks.npz), the device routine under the emulator against the oracle, and -- on the GPU -- unc_dtw_batch
 through the Python classes against the oracle.  Bit-exact: path, score, mean score."""
 import ctypes as C
 
@@ -44,25 +44,35 @@ def _oracle(M, kind, sub, w, means, km):
     return p[:2 * n.value].reshape(-1, 2).copy(), s.value
 
 
-@pytest.mark.skipif(not orclib.ref_available(), reason="oracle/_ref is built only where /root/reference exists")
-def test_oracle_dtw_equals_the_reference_classes():
-    R = orclib.ref()
-    R.ref_dtw.argtypes = [C.c_int, C.c_int, C.c_float, C.c_float, C.c_float, f32p, C.c_uint32, u16p, C.c_uint32, u64p, u64p, f32p, f32p]
-    M = _template_model()
+def dtw_problems():
+    """400 random problems: (kind, sub, weights, event means, k-mers)"""
     rng = np.random.default_rng(1)
     for t in range(400):
         nr, nc = int(rng.integers(1, 70)), int(rng.integers(1, 70))
         kind, sub, w = int(rng.integers(0, 2)), int(rng.integers(0, 3)), PRESETS[int(rng.integers(0, 4))]
         means, km = _problem(rng, nr, nc, rng.random() < 0.7)
-        want = np.zeros(2 * (nr + nc), np.uint64)
-        n, s, ms = C.c_uint64(), C.c_float(), C.c_float()
-        R.ref_dtw(kind, sub, w[0], w[1], w[2], means.ctypes.data_as(f32p), nc, km.ctypes.data_as(u16p), nr, want.ctypes.data_as(u64p),
-                  C.byref(n), C.byref(s), C.byref(ms))
+        yield kind, sub, w, means, km
+
+
+def test_oracle_dtw_equals_the_reference_classes():
+    """Against the paths and scores of the reference's DTWr94p / DTWr94d on the same problems
+    (tests/golden/reference_checks.npz, tools/make_reference_checks_golden.py)."""
+    g = np.load(orclib.REFERENCE_CHECKS_NPZ)
+    want_path, want_len = g["dtw/path"].astype(np.uint64), g["dtw/path_len"]
+    want_score, want_mean = g["dtw/score"], g["dtw/mean_score"]
+    assert len(want_len) == 400
+    M = _template_model()
+    at = 0
+    for t, (kind, sub, w, means, km) in enumerate(dtw_problems()):
+        n = int(want_len[t])
+        want = want_path[at:at + 2 * n]
+        at += 2 * n
         path, score = _oracle(M, kind, sub, w, means, km)
-        assert len(path) == n.value and score == s.value and np.array_equal(path.ravel(), want[:2 * n.value]), (t, kind, sub, nr, nc)
-        assert np.float32(score) / np.float32(len(path)) == np.float32(ms.value)
+        assert len(path) == n and score == want_score[t] and np.array_equal(path.ravel(), want), (t, kind, sub, len(km), len(means))
+        assert np.float32(score) / np.float32(len(path)) == want_mean[t]
         if kind == 1 and all(float(x).is_integer() for x in w):
             assert score == int(score)                 # abs() of the truncated difference: whole numbers (integer weights)
+    assert at == len(want_path)
 
 
 def _emul(kind, sub, w, probs, n_threads):

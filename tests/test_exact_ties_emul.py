@@ -77,41 +77,27 @@ def test_exact_ties_on_a_small_buffer_and_odd_cta_shapes(setup):
         O.lib.orc_set_child_sort(0)
 
 
-BOTH_EXACT = r"""
-import sys, ctypes as C
-sys.path[:0] = [%r, %r]
-import numpy as np, orclib, emulib, synth, synthdata
-prefix, g = synthdata.get_index("g4m7")
-R = orclib.ref()                                  # the reference's own code, unmodified (pdqsort as vendored)
-assert R.ref_load(prefix.encode(), b"default") == 0
-sig, _ = synth.reads(g, 600, 4000, seed=7, frac_random=0.15)
-ids = [36, 588, 589, 590]                             # 36: tie order decides a seed; 589: depends on what 588 leaves set
-sigs = [np.ascontiguousarray(sig[i], np.float32) for i in ids]
-n = len(ids)
-flat = np.concatenate(sigs)
-offs, lens = (np.arange(n) * 4000).astype(np.uint64), np.full(n, 4000, np.uint32)
-ref = (orclib.RefPaf * n)()
-R.ref_map_batch_mt(orclib.fp(flat), offs.ctypes.data_as(orclib.u64p), lens.ctypes.data_as(orclib.u32p), n, 1, ref)   # ONE Mapper
-E = emulib.Emu(prefix)
-E.set_tie_order(1)
-exact, _, n_re, _ = E.map_ordered(sigs)
-E.set_tie_order(0)
-plain = E.map_batch(sigs)[0]
-want = [orclib.paf_tuple(r) for r in ref]
-print("EXACT-DIFF", [ids[i] for i in range(n) if emulib.paf_tuple(exact[i]) != want[i]], "REMAPPED", n_re)
-print("PLAIN-DIFF", [ids[i] for i in range(n) if emulib.paf_tuple(plain[i]) != want[i]])
-"""
-
-
 def test_both_exact_modes_together_equal_the_unmodified_references_long_lived_mapper():
-    """No oracle in between: ONE Mapper of the reference's own code (oracle/_ref, pdqsort as vendored) over four reads in
-    order, against the emulated exact-ties kernel driven by the ordered-mode host logic.  The default configuration
-    differs on exactly the two reads DESIGN.md section 2 explains (36: tie order, 589: flags left by 588)."""
-    import sys
-    if not orclib.ref_available():
-        pytest.skip("oracle/_ref not built")
-    out = orclib.run_in_subprocess(BOTH_EXACT % (os.path.join(ROOT, "tests"), os.path.join(ROOT, "tools")), timeout=900)
-    assert "EXACT-DIFF [] REMAPPED 1" in out and "PLAIN-DIFF [36, 589]" in out, out
+    """No oracle in between: ONE Mapper of the reference's own code (oracle/_ref, pdqsort as vendored; its records stored
+    in tests/golden/reference_checks.json) over four reads in order, against the emulated exact-ties kernel driven by the
+    ordered-mode host logic.  The default configuration differs on exactly the two reads DESIGN.md section 2 explains
+    (36: tie order, 589: flags left by 588)."""
+    import synth
+    import synthdata
+    want = orclib.reference_checks("divergences")["one_mapper_36_588_589_590"]
+    prefix, g = synthdata.get_index("g4m7")
+    sig, _ = synth.reads(g, 600, 4000, seed=7, frac_random=0.15)
+    ids = [36, 588, 589, 590]                             # 36: tie order decides a seed; 589: depends on what 588 leaves set
+    sigs = [np.ascontiguousarray(sig[i], np.float32) for i in ids]
+    E = emulib.Emu(prefix)
+    E.set_tie_order(1)
+    try:
+        exact, _, n_re, _ = E.map_ordered(sigs)
+    finally:
+        E.set_tie_order(0)
+    plain = E.map_batch(sigs)[0]
+    assert [ids[i] for i in range(4) if list(emulib.paf_tuple(exact[i])) != want[i]] == [] and n_re == 1
+    assert [ids[i] for i in range(4) if list(emulib.paf_tuple(plain[i])) != want[i]] == [36, 589]
 
 
 def test_streaming_path_with_exact_ties(setup):

@@ -2,10 +2,10 @@
 
 Pins, in this order:
   * the oracle's self_align against digests of the reference's own C++ self_align
-    (tests/golden/self_align_golden.json, tools/make_selfalign_golden.py) and, live, against oracle/_ref;
+    (tests/golden/self_align_golden.json, tools/make_selfalign_golden.py and tests/golden/reference_checks.json);
   * uncalled_b200.index_params against (a) the `.uncl` file the reference SHIPS with its example index,
     (b) lines written by the real `uncalled index` for seeded genomes (tests/golden/synth_uncl.json) and
-    (c) multi-preset files written by the reference's IndexParameterizer imported from /root/reference
+    (c) multi-preset files written by the reference's own IndexParameterizer
     (tests/golden/uncl_presets.json, tools/make_uncl_presets_golden.py) -- character for character."""
 import hashlib
 import json
@@ -59,26 +59,14 @@ def test_oracle_self_align_matches_reference_digest(row):
     assert sha(off) == row["offsets_sha256"] and sha(val) == row["values_sha256"]
 
 
-LIVE = r"""
-import sys
-sys.path[:0] = [%r, %r]
-import numpy as np, orclib, synthdata
-prefix = synthdata.get_index("g200k")[0]
-for sd in (1, 7, 250):
-    a, b = orclib.ref_self_align(prefix, sd), orclib.self_align(prefix, sd)
-    assert np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1]), sd
-print("LIVE-OK")
-"""
-
-
 def test_oracle_self_align_matches_ref_library_live():
-    import subprocess
+    """Against the reference's own self_align (oracle/_ref) on the 200 kb index at three sampling distances; its
+    digests are stored in tests/golden/reference_checks.json (tools/make_reference_checks_golden.py)."""
     import orclib
-    if not orclib.ref_available():
-        pytest.skip("oracle/_ref not built")
-    r = subprocess.run([sys.executable, "-c", LIVE % (os.path.join(ROOT, "tests"), os.path.join(ROOT, "tools"))],
-                       capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0 and "LIVE-OK" in r.stdout, r.stdout + r.stderr
+    from make_reference_checks_golden import sa_digest
+    gold = orclib.reference_checks("self_align_g200k")
+    for sd in (1, 7, 250):
+        assert sa_digest(*paths_of("g200k", sd)) == gold[str(sd)], sd
 
 
 def test_sample_distance_rules():

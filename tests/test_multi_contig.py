@@ -1,8 +1,8 @@
 """Mapping against a reference with SEVERAL sequences (and ambiguous bases): bns_pos2rid / translate_loc
 (reference submods/bwa/bntseq.c:354-368, src/bwa_index.hpp:213-220) turn an FM coordinate into (contig, offset).
 The index is built end to end by the product's own `uncalled index` (FM builder + self-alignments on the emulated device
-+ parameter search); reads from every contig and both strands are mapped by the emulated kernels, the oracle and -- when
-it is built -- the reference's own code."""
++ parameter search); reads from every contig and both strands are mapped by the emulated kernels, the oracle and the
+reference's own code (its records stored in tests/golden/reference_checks.json)."""
 import os
 import sys
 
@@ -60,14 +60,5 @@ def test_reads_map_to_the_right_contig(tmp_path):
     assert len(hit) >= 7 and len(set(h[0] for h in hit)) == 3 and all(lens[rid] == rl for rid, rl in hit)
     assert [r.rid for r in recs[:9] if r.mapped] == sorted(r.rid for r in recs[:9] if r.mapped)   # reads 0-2 -> chrA, 3-5 -> chrB, ...
     assert not recs[-1].mapped
-    if orclib.ref_available():                       # the oracle against the reference's own Mapper on this index
-        np.save(os.path.join(str(tmp_path), "sigs.npy"), np.stack(sigs))
-        code = ("import sys; sys.path[:0]=[%r]; import numpy as np, ctypes as C, orclib\n"
-                "R = orclib.ref(); assert R.ref_load(%r.encode(), b'default') == 0\n"
-                "O = orclib.Oracle(%r)\n"
-                "for s in np.load(%r):\n"
-                "    s = np.ascontiguousarray(s, np.float32); out = orclib.RefPaf()\n"
-                "    R.ref_map_read(orclib.fp(s), len(s), C.byref(out))\n"
-                "    assert orclib.paf_tuple(out) == orclib.paf_tuple(O.map_read(s))\n"
-                "print('OK')") % (os.path.join(ROOT, "tests"), prefix, prefix, os.path.join(str(tmp_path), "sigs.npy"))
-        assert "OK" in orclib.run_in_subprocess(code)
+    want = orclib.reference_checks("multi_contig")["paf"]       # the reference's own Mapper on this index
+    assert [list(orclib.paf_tuple(O.map_read(np.ascontiguousarray(s, np.float32)))) for s in sigs] == want

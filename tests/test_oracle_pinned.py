@@ -1,11 +1,10 @@
 """CPU tier: the oracle (oracle/unc_oracle.c) is pinned against (a) golden vectors produced by
-the real reference (tests/golden, tools/make_golden.py) and (b) oracle/_ref -- the reference's
-own mapper sources compiled unmodified -- when that library is present."""
+the real reference (tests/golden, tools/make_golden.py) and (b) records of the reference's own mapper sources
+compiled unmodified (oracle/_ref) on seeded synthetic reads (tests/golden/reference_checks.json)."""
 import ctypes as C
 import json
 import os
 import sys
-import textwrap
 
 import numpy as np
 import pytest
@@ -74,84 +73,41 @@ def test_empty_and_tiny_reads(O):
         assert not r.mapped and r.rd_len == int(np.float32(n) * (np.float32(450) / np.float32(4000)))
 
 
-@pytest.mark.skipif(not orclib.ref_available(), reason="oracle/_ref not built (needs /root/reference)")
+def _keys(recs):
+    return [[int(v) for v in orclib.paf_tuple(r)] for r in recs]
+
+
 def test_oracle_equals_unmodified_reference_on_synthetic_reads():
-    """Bit-for-bit PAF agreement with the reference's own Mapper (fresh Mapper per read) on
-    seeded synthetic reads, incl. reads that never map.  Runs in a child: _ref is static."""
-    code = textwrap.dedent("""
-        import sys, ctypes as C, numpy as np
-        sys.path.insert(0, %r); sys.path.insert(0, %r); sys.path.insert(0, %r)
-        import orclib as o, synth, synthdata
-        prefix, g = synthdata.get_index("g200k")
-        sig, truth = synth.reads(g, 96, 4000, seed=11)
-        O = o.Oracle(prefix)
-        R = o.ref(); R.ref_load(prefix.encode(), b"default")
-        offs = np.arange(96, dtype=np.uint64) * 4000
-        po = O.map_batch(sig.ravel(), offs, np.full(96, 4000, np.uint32), 4)
-        bad = 0
-        for i in range(96):
-            out = o.RefPaf()
-            R.ref_map_read(o.fp(sig[i]), 4000, C.byref(out))
-            if o.paf_tuple(po[i]) != o.paf_tuple(out): bad += 1
-        # events / normalisation / model straight from the reference classes
-        ev = np.zeros(4001, np.float32); st = np.zeros(4001, np.uint32); ln = np.zeros(4001, np.uint32); mel = C.c_float()
-        ne = R.ref_get_events(o.fp(sig[0]), 4000, o.fp(ev), st.ctypes.data_as(o.u32p), ln.ctypes.data_as(o.u32p), C.byref(mel))
-        m, s, l, omel = O.detect(sig[0])
-        assert ne == len(m) and np.array_equal(ev[:ne], m) and np.float32(mel.value) == omel
-        nm = np.zeros(ne, np.float32); R.ref_normalize(o.fp(m), ne, o.fp(nm))
-        assert np.array_equal(nm, O.normalize(m))
-        assert all(R.ref_match_prob(float(e), k) == O.lib.orc_match_prob(C.byref(O.model), float(e), k)
-                   for e in (61.5, 90.25, 118.0) for k in range(1024))
-        assert all(R.ref_prob_thresh(b) == O.lib.orc_prob_thresh(O.idx, b) or
-                   (np.isnan(R.ref_prob_thresh(b)) and np.isnan(O.lib.orc_prob_thresh(O.idx, b))) for b in range(64))
-        print("MISMATCHES", bad, "MAPPED", sum(r.mapped for r in po))
-    """ % (ROOT, os.path.join(ROOT, "tests"), os.path.join(ROOT, "tools")))
-    out = orclib.run_in_subprocess(code, timeout=900)
-    assert "MISMATCHES 0" in out, out
+    """Bit-for-bit PAF agreement with the reference's own Mapper (fresh Mapper per read) on seeded synthetic reads, incl.
+    reads that never map; events, normalisation, model and thresholds as the reference classes give them.  The
+    reference's results are stored in tests/golden/reference_checks.{json,npz} (tools/make_reference_checks_golden.py)."""
+    import synth
+    import synthdata
+    gold, g = orclib.reference_checks("synthetic_reads"), np.load(orclib.REFERENCE_CHECKS_NPZ)
+    prefix, genome = synthdata.get_index("g200k")
+    sig, _ = synth.reads(genome, 96, 4000, seed=11)
+    O = orclib.Oracle(prefix)
+    offs = np.arange(96, dtype=np.uint64) * 4000
+    po = O.map_batch(sig.ravel(), offs, np.full(96, 4000, np.uint32), 4)
+    assert _keys(po) == gold["paf"]
+    assert 0 < sum(r.mapped for r in po) < 96
+    m, s, l, mel = O.detect(sig[0])
+    assert np.array_equal(m, g["synthetic_reads/ev_mean"]) and np.array_equal(s, g["synthetic_reads/ev_start"])
+    assert np.array_equal(l, g["synthetic_reads/ev_len"]) and mel == g["synthetic_reads/mean_event_len"]
+    assert np.array_equal(O.normalize(m), g["synthetic_reads/normed"])
+    probs = np.array([[O.lib.orc_match_prob(C.byref(O.model), e, k) for k in range(1024)] for e in (61.5, 90.25, 118.0)], np.float32)
+    assert np.array_equal(probs, g["synthetic_reads/match_prob"])
+    thr = np.array([O.lib.orc_prob_thresh(O.idx, b) for b in range(64)], np.float32)
+    assert np.array_equal(thr, g["synthetic_reads/prob_thresh"], equal_nan=True)
 
 
-T1_ORDER = r"""
-import sys, ctypes as C
-sys.path[:0] = [%r, %r]
-import numpy as np, orclib, synth, synthdata
-prefix, g = synthdata.get_index("g4m7")
-R = orclib.ref()
-assert R.ref_load(prefix.encode(), b"default") == 0
-O = orclib.Oracle(prefix)
-sig, _ = synth.reads(g, 600, 4000, seed=7, frac_random=0.15)       # the 600-read set DESIGN.md section 2 quotes
-lo, hi = 575, 595
-sub = sig[lo:hi]
-n = hi - lo
-flat = np.ascontiguousarray(sub.reshape(-1))
-offs, lens = (np.arange(n) * 4000).astype(np.uint64), np.full(n, 4000, np.uint32)
-ref = (orclib.RefPaf * n)()
-R.ref_map_batch_mt(orclib.fp(flat), offs.ctypes.data_as(orclib.u64p), lens.ctypes.data_as(orclib.u32p), n, 1, ref)
-carried = O.map_reads_one_mapper(flat, offs, lens)
-fresh = O.map_batch(flat, offs, lens, threads=4)
-assert [orclib.paf_tuple(r) for r in ref] == [orclib.paf_tuple(r) for r in carried]
-print("CARRY-DIFF", [lo + i for i in range(n) if orclib.paf_tuple(fresh[i]) != orclib.paf_tuple(carried[i])])
-# tie order: fresh Mapper on both sides, reads 30..39
-d = []
-for i in range(30, 40):
-    s = np.ascontiguousarray(sig[i], np.float32)
-    out = orclib.RefPaf()
-    R.ref_map_read(orclib.fp(s), len(s), C.byref(out))
-    a, b = orclib.paf_tuple(out), orclib.paf_tuple(O.map_read(s))
-    if a != b:
-        d.append((i, a[5], a[10], b[5], b[10]))
-print("TIE-DIFF", d)
-# ... and with the reference's pdqsort restated in the oracle (orc_set_child_sort(1)) nothing differs any more, here and on
-# reads of a second set that the stable order maps differently
-O.lib.orc_set_child_sort(1)
-b, _ = synth.reads(g, 2400, 4000, seed=123, frac_random=0.15)
-for s in [sig[i] for i in range(30, 40)] + [b[i] for i in (64, 137, 1395, 1598, 1971)]:
-    s = np.ascontiguousarray(s, np.float32)
-    out = orclib.RefPaf()
-    R.ref_map_read(orclib.fp(s), len(s), C.byref(out))
-    assert orclib.paf_tuple(out) == orclib.paf_tuple(O.map_read(s))
-O.lib.orc_set_child_sort(0)
-print("PDQ-OK")
-"""
+def _g4m7_sets():
+    import synth
+    import synthdata
+    prefix, g = synthdata.get_index("g4m7")
+    a, _ = synth.reads(g, 600, 4000, seed=7, frac_random=0.15)       # the 600-read set DESIGN.md section 2 quotes
+    b, _ = synth.reads(g, 2400, 4000, seed=123, frac_random=0.15)
+    return prefix, a, b
 
 
 def test_the_two_documented_divergences_and_nothing_else():
@@ -161,51 +117,44 @@ def test_the_two_documented_divergences_and_nothing_else():
     (2) Tie order: the reference sorts children with pdqsort (unstable); of reads 30..39 mapped by FRESH Mappers on both
     sides, read 36 ends one seed longer in the reference (matches 55 / rf_en 1749657 against 54 / 1749656) and the other
     nine are identical; with pdqsort itself restated in the oracle (orc_set_child_sort(1)) all of them, and five reads of a
-    second set that the stable order maps differently, are identical to the unmodified reference."""
-    import subprocess
-    import orclib
-    if not orclib.ref_available():
-        pytest.skip("oracle/_ref not built")
-    r = subprocess.run([sys.executable, "-c", T1_ORDER % (os.path.join(ROOT, "tests"), os.path.join(ROOT, "tools"))],
-                       capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0, r.stdout[-1500:] + r.stderr[-1500:]
-    assert "CARRY-DIFF [589]" in r.stdout and "TIE-DIFF [(36, 55, 1749657, 54, 1749656)]" in r.stdout, r.stdout
-    assert "PDQ-OK" in r.stdout
-
-
-STABLE = r"""
-import sys, ctypes as C
-sys.path[:0] = [%r, %r]
-import numpy as np, orclib, synth, synthdata
-prefix, g = synthdata.get_index("g4m7")
-R = orclib.ref(stable_sort=True)
-assert R.ref_load(prefix.encode(), b"default") == 0
-O = orclib.Oracle(prefix)
-a, _ = synth.reads(g, 600, 4000, seed=7, frac_random=0.15)
-b, _ = synth.reads(g, 2400, 4000, seed=123, frac_random=0.15)
-picks = [a[i] for i in range(30, 40)] + [b[i] for i in (64, 137, 1395, 1598)]   # incl. five reads the pdqsort build maps differently
-for k, s in enumerate(picks):
-    s = np.ascontiguousarray(s, np.float32)
-    out = orclib.RefPaf()
-    R.ref_map_read(orclib.fp(s), len(s), C.byref(out))
-    assert orclib.paf_tuple(out) == orclib.paf_tuple(O.map_read(s)), k
-print("STABLE-OK")
-"""
+    second set that the stable order maps differently, are identical to the unmodified reference.  The reference's
+    records are stored in tests/golden/reference_checks.json (tools/make_reference_checks_golden.py)."""
+    gold = orclib.reference_checks("divergences")
+    prefix, sig, b = _g4m7_sets()
+    O = orclib.Oracle(prefix)
+    lo, hi = 575, 595
+    n = hi - lo
+    flat = np.ascontiguousarray(sig[lo:hi].reshape(-1))
+    offs, lens = (np.arange(n) * 4000).astype(np.uint64), np.full(n, 4000, np.uint32)
+    carried = _keys(O.map_reads_one_mapper(flat, offs, lens))
+    fresh = _keys(O.map_batch(flat, offs, lens, threads=4))
+    assert carried == gold["one_mapper_575_595"]
+    assert [lo + i for i in range(n) if fresh[i] != carried[i]] == [589]
+    mine = _keys(O.map_read(np.ascontiguousarray(sig[i], np.float32)) for i in range(30, 40))
+    d = [(30 + j, a[5], a[10], m[5], m[10]) for j, (a, m) in enumerate(zip(gold["fresh_30_40"], mine)) if a != m]
+    assert d == [(36, 55, 1749657, 54, 1749656)]
+    O.lib.orc_set_child_sort(1)
+    try:
+        picks = [sig[i] for i in range(30, 40)] + [b[i] for i in (64, 137, 1395, 1598, 1971)]
+        got = _keys(O.map_read(np.ascontiguousarray(s, np.float32)) for s in picks)
+    finally:
+        O.lib.orc_set_child_sort(0)
+    assert got == gold["fresh_30_40"] + gold["fresh_second_set"]
 
 
 def test_reference_with_a_stable_child_sort_agrees_on_every_read():
-    """The tie-order divergence isolated: oracle/_ref/libuncalled_ref_stable.so is the reference's own code with the
-    vendored pdqsort shadowed by std::stable_sort (oracle/ref_build/stubs_stable/pdqsort.h).  It agrees with the oracle
-    on the reads that the unmodified reference maps differently (measured once over 2400 bench-like reads: 7 differ with
-    pdqsort, 0 with the stable sort) -- the sort's instability is the only source of difference."""
-    import subprocess
-    import orclib
-    if not (orclib.ref_available() and os.path.exists(os.path.join(orclib.ORACLE_DIR, "_ref", "libuncalled_ref_stable.so"))):
-        pytest.skip("oracle/_ref not built")
-    r = subprocess.run([sys.executable, "-c", STABLE % (os.path.join(ROOT, "tests"), os.path.join(ROOT, "tools"))],
-                       capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0 and "STABLE-OK" in r.stdout, r.stdout[-1500:] + r.stderr[-1500:]
-
+    """The tie-order divergence isolated: the reference's own code with the vendored pdqsort shadowed by std::stable_sort
+    (oracle/ref_build/stubs_stable/pdqsort.h; its records stored in tests/golden/reference_checks.json) agrees with the
+    oracle on the reads that the unmodified reference maps differently (measured once over 2400 bench-like reads: 7 differ
+    with pdqsort, 0 with the stable sort) -- the sort's instability is the only source of difference."""
+    gold = orclib.reference_checks("stable_sort")
+    prefix, a, b = _g4m7_sets()
+    O = orclib.Oracle(prefix)
+    picks = [a[i] for i in range(30, 40)] + [b[i] for i in (64, 137, 1395, 1598)]
+    got = _keys(O.map_read(np.ascontiguousarray(s, np.float32)) for s in picks)
+    for k, (w, m) in enumerate(zip(gold["fresh"], got)):
+        assert w == m, k
+    assert len(got) == len(gold["fresh"]) == 14
 
 
 def test_oracle_matches_reference_made_paf_golden_in_both_sort_modes():

@@ -1,7 +1,7 @@
 """The oracle's restatement of the STREAMING path (EventProfiler, streaming Normalizer, chunked
 process_chunk / map_chunk) against (a) committed results of the reference's own streaming path
 (tests/golden/stream_golden.json, made by tools/make_stream_golden.py from oracle/_ref) and
-(b) oracle/_ref itself when it is present."""
+(b) the same on fresh synthetic reads (tests/golden/reference_checks.json)."""
 import json
 import os
 import sys
@@ -37,33 +37,17 @@ def test_example_read_streams_like_uncalled_map_ord():
     assert p[0] == 1 and p[1] == 0 and p[6:11] == [67, 41, 67, 6948, 6977] and p[5] == 29
 
 
-LIVE = r"""
-import ctypes as C, sys
-sys.path[:0] = [%r, %r]
-import numpy as np, orclib, synth, synthdata
-prefix, g = synthdata.get_index("g200k")
-R = orclib.ref()
-assert R.ref_load(prefix.encode(), b"default") == 0
-O = orclib.Oracle(prefix)
-sig, _ = synth.reads(g, 10, 9000, seed=77, frac_random=0.3)
-for i in range(10):
-    s = np.ascontiguousarray(sig[i], np.float32)
-    for ct, mc in ((0.1125, 1000000), (0.1125, 7), (0.25, 3)):
-        out, nu, en = orclib.RefPaf(), C.c_uint32(), C.c_int32()
-        R.ref_stream_read(orclib.fp(s), len(s), ct, mc, C.byref(out), C.byref(nu), C.byref(en))
-        rec, nu2, en2 = O.stream_read(s, int(np.float32(ct) * np.float32(4000.0)), mc)
-        assert (orclib.paf_tuple(out), nu.value, en.value) == (orclib.paf_tuple(rec), nu2, en2), (i, ct, mc)
-print("LIVE-OK")
-"""
-
-
 def test_stream_port_matches_ref_library_live():
-    """bit-for-bit against oracle/_ref on fresh reads; in its own process because the reference keeps
-    its FM index in process-global statics (one index per process)."""
-    import subprocess
+    """bit-for-bit against the reference's own streaming Mapper (oracle/_ref) on fresh reads; its records are stored in
+    tests/golden/reference_checks.json (tools/make_reference_checks_golden.py)."""
     import orclib
-    if not orclib.ref_available():
-        pytest.skip("oracle/_ref not built")
-    r = subprocess.run([sys.executable, "-c", LIVE % (os.path.join(ROOT, "tests"), os.path.join(ROOT, "tools"))],
-                       capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0 and "LIVE-OK" in r.stdout, r.stdout + r.stderr
+    import synth
+    import synthdata
+    rows = orclib.reference_checks("stream")["rows"]
+    assert len(rows) == 30
+    prefix, g = synthdata.get_index("g200k")
+    O = orclib.Oracle(prefix)
+    sig, _ = synth.reads(g, 10, 9000, seed=77, frac_random=0.3)
+    for row in rows:
+        rec, nu, en = O.stream_read(np.ascontiguousarray(sig[row["read"]], np.float32), _chunk_len(row["chunk_time"]), row["max_chunks"])
+        assert (list(orclib.paf_tuple(rec)), nu, en) == (row["paf"], row["chunks"], row["ended"]), row

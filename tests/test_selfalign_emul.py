@@ -62,10 +62,7 @@ def test_repeats_short_and_ambiguous_sequences(tmp_path):
         assert np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1]), sd
         lens = np.diff(a[0].astype(np.int64))
         assert lens.max() > 1000 and lens.min() >= 1           # repeats: far beyond the staging depth of 48
-    if orclib.ref_available():                                  # and the oracle against the reference's own code, live
-        code = ("import sys; sys.path[:0]=[%r]; import numpy as np, orclib\n"
-                "for sd in (1, 3):\n"
-                "    a, b = orclib.ref_self_align(%r, sd), orclib.self_align(%r, sd)\n"
-                "    assert np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1])\n"
-                "print('OK')") % (os.path.join(ROOT, "tests"), prefix, prefix)
-        assert "OK" in orclib.run_in_subprocess(code)
+    from make_reference_checks_golden import sa_digest
+    gold = orclib.reference_checks("self_align_repeats")       # and the oracle against the reference's own self_align
+    for sd in (1, 3):
+        assert sa_digest(*orclib.self_align(prefix, sd)) == gold[str(sd)], sd
