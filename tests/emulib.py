@@ -59,23 +59,23 @@ def make_descs(lens, dtype=0, cal=(1.0, 0.0, 1.0)):
     return d
 
 
-def build(extra_flags=(), tag=""):
-    """Compiles the device source for the host.  extra_flags/tag build a variant (e.g. -DK2_LEAN_B) next to the default."""
+def build():
+    """Compiles the device source for the host."""
     src = os.path.join(EMUL_DIR, "emul_main.cpp")
-    out = os.path.join(EMUL_DIR, "libunc_emul%s.so" % tag)
+    out = os.path.join(EMUL_DIR, "libunc_emul.so")
     deps = [src, os.path.join(EMUL_DIR, "warp_emul.hpp")] + \
            [os.path.join(ROOT, "uncalled_b200", "csrc", f) for f in
             ("unc_device.cuh", "unc_k2v2.cuh", "unc_dtw.cuh", "unc_k1.cuh", "unc_stream.cuh", "unc_stream_logic.hpp", "unc_ordered_logic.hpp", "unc_pdqsort.cuh", "unc_warp.cuh", "unc_host_index.hpp", "unc_host_params.hpp",
              "unc_selfalign.cuh", "unc_selfalign_host.hpp")]
     if os.path.exists(out) and all(os.path.getmtime(out) >= os.path.getmtime(d) for d in deps):
         return out
-    subprocess.run(["g++", "-O2", "-g", "-std=c++17", "-ffp-contract=off", "-DUNC_EMUL", "-DK2_MAXSEG=16u", "-fPIC", "-shared",
-                    "-I" + EMUL_DIR, "-I" + os.path.join(ROOT, "uncalled_b200", "csrc"), "-o", out, src] + list(extra_flags),
+    subprocess.run(["g++", "-O2", "-g", "-std=c++17", "-ffp-contract=off", "-DUNC_EMUL", "-fPIC", "-shared",
+                    "-I" + EMUL_DIR, "-I" + os.path.join(ROOT, "uncalled_b200", "csrc"), "-o", out, src],
                    check=True, capture_output=True)
     return out
 
 
-_libs = {}
+_lib = None
 
 
 def _bind(L):
@@ -106,16 +106,17 @@ def _bind(L):
     return L
 
 
-def lib(extra_flags=(), tag=""):
-    """The emulator library; (extra_flags, tag) select a compile-time variant of the device source."""
-    if tag not in _libs:
-        _libs[tag] = _bind(C.CDLL(build(extra_flags, tag)))
-    return _libs[tag]
+def lib():
+    """The emulator library."""
+    global _lib
+    if _lib is None:
+        _lib = _bind(C.CDLL(build()))
+    return _lib
 
 
 class Emu:
-    def __init__(self, prefix, preset="default", extra_flags=(), tag=""):
-        self.L = lib(extra_flags, tag)
+    def __init__(self, prefix, preset="default"):
+        self.L = lib()
         self.idx = self.L.emu_index_load(prefix.encode(), preset.encode(), MODEL_TABLE.encode())
         if not self.idx:
             raise RuntimeError("emu_index_load failed")

@@ -121,14 +121,13 @@ def test_streaming_path_with_exact_ties(setup):
         O.lib.orc_set_child_sort(0)
 
 
-def test_both_exact_modes_in_the_combined_prototype_build():
-    """The compile-time prototypes of the mapper (no tracker warp, lean extension loop, ...: DESIGN.md section 7) keep the
-    ordered-mode flag handling and the exact-ties sort working -- whichever of them becomes the shipped configuration."""
+def test_both_exact_modes_on_a_small_buffer_and_a_5_warp_cta():
+    """Ordered mode and exact ties together, against one Mapper of the oracle with the reference's child sort: max_paths
+    300 and a 5-warp CTA.  The sources_added_ words the four reads leave behind match too."""
     import synth
     import synthdata
-    flags = ("-DK2_TRK_INLINE", "-DK2_LEAN_B", "-DK2_PAR_E", "-DK2_SCAN2", "-DK2_PF2", "-DK2_DFUSE")
     prefix, g = synthdata.get_index("g200k")
-    E, O = emulib.Emu(prefix, extra_flags=flags, tag="_all"), orclib.Oracle(prefix)
+    E, O = emulib.Emu(prefix), orclib.Oracle(prefix)
     E.params.max_paths = O.params.max_paths = 300
     sig, _ = synth.reads(g, 40, 2000, seed=21, frac_random=0.4)
     sigs = [np.ascontiguousarray(sig[i], np.float32) for i in (5, 6, 0, 1)]

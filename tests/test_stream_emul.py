@@ -46,6 +46,7 @@ def test_reads_following_each_other_on_shared_channels(g200k):
     sigs = [sig[i][:5000 - 37 * i] for i in range(4)] + [sig[0][:300]]      # the last one is shorter than a chunk
     st = _check(E, O, sigs, 2, 450)
     assert (2, 0) in st
+    _check(E, O, [sig[i] for i in range(3)], 3, 450, max_chunks=4, n_warps=3)   # one read per channel, a 3-warp CTA
 
 
 def test_max_chunks_and_one_second_chunks(g200k):
@@ -55,19 +56,6 @@ def test_max_chunks_and_one_second_chunks(g200k):
     st = _check(E, O, [sig[i] for i in range(5)], 5, 450, max_chunks=4)
     assert (3, 1) in st                                  # gave up when the signal (max_chunks) ran out: ended
     _check(E, O, [sig[i][:4500] for i in range(2)], 2, 4000, n_warps=2)   # chunk_time 1.0 s, a 2-warp CTA
-
-
-@pytest.mark.parametrize("flags,tag", [(("-DK2_TRK_INLINE", "-DK2_LEAN_B", "-DK2_PAR_E", "-DK2_SCAN2", "-DK2_PF2", "-DK2_DFUSE"), "_all")])
-def test_tracker_inline_variant_streams_identically(g200k, flags, tag):
-    """-DK2_TRK_INLINE keeps the seed tracker's state in shared memory between events and in the channel's
-    DevMapState between chunks: same results chunk by chunk (alone and with the other prototypes)."""
-    prefix, g = g200k
-    E = emulib.Emu(prefix, extra_flags=flags, tag=tag)
-    O = orclib.Oracle(prefix)
-    sig, _ = synth.reads(g, 4, 5000, seed=5, frac_random=0.3)
-    st = _check(E, O, [sig[i][:5000 - 37 * i] for i in range(4)], 2, 450)
-    assert (2, 0) in st
-    _check(E, O, [sig[i] for i in range(3)], 3, 450, max_chunks=4, n_warps=3)
 
 
 def test_max_events_and_small_path_buffer(g200k):

@@ -2,7 +2,7 @@
 {10000, 1000, 300, 77}, max_events in {30000, 200}, 2..16-warp CTAs on the 200 kb and 1 Mb indexes -- the default kernel
 against the oracle (stable order, new Mapper per read), and the exact-ties kernel under the ordered-mode host logic
 against the oracle's pdqsort one-Mapper chain; PAF fields and the children / sources / seeds / clusters counters.
-    python tools/emul_sweep.py [seed [configs per index [all]]]     (`all`: the combined prototype build)"""
+    python tools/emul_sweep.py [seed [configs per index]]"""
 import sys, time
 import os
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -14,11 +14,7 @@ key = lambda r, P: (P.paf_tuple(r), cnt(r))
 bad = 0; total = 0; t0 = time.time()
 for name in ("g200k", "g1m"):
     prefix, g = synthdata.get_index(name)
-    if len(sys.argv) > 3 and sys.argv[3] == "all":     # the combined prototype build (DESIGN.md section 7)
-        E = emulib.Emu(prefix, extra_flags=("-DK2_TRK_INLINE", "-DK2_LEAN_B", "-DK2_PAR_E", "-DK2_SCAN2", "-DK2_PF2", "-DK2_DFUSE",
-                                            "-DK2_BMATCH"), tag="_everything")
-    else:
-        E = emulib.Emu(prefix)
+    E = emulib.Emu(prefix)
     O = orclib.Oracle(prefix)
     for rep in range(int(sys.argv[2]) if len(sys.argv) > 2 else 10):
         mp = int(rng.choice([10000, 1000, 300, 77])); me = int(rng.choice([30000, 30000, 200]))

@@ -32,11 +32,7 @@ static_assert(sizeof(DevReadDesc) == 32, "DevReadDesc layout");
 #endif
 #define K2_MIN_CTAS_V1 (K2_WARPS > 8 ? 1 : 2)    /* first structure (exact-ties kernels): 127 registers */
 #define K2_THREADS (K2_WARPS * 32)
-#ifdef K2_TRK_INLINE
-static_assert(K2_WARPS >= 1 && K2_WARPS <= K2_MAXSEG, "worker warps (all of them) must fit the sort segments");
-#else
 static_assert(K2_WARPS >= 2 && K2_WARPS - 1 <= K2_MAXSEG, "worker warps must fit the sort segments");
-#endif
 
 __global__ void k_kmer_ranges(DevIndex ix, uint2 *out) {
     u32 k = blockIdx.x * blockDim.x + threadIdx.x;
@@ -86,26 +82,9 @@ __global__ void __launch_bounds__(128) k1_norm(DevBatch B, DevParams p) {
 // of the CTA cooperate on every event of the read (chained scans through shared memory).
 #define K2_MAP_KERNEL(NAME, EXACT, FLAGS)                                                                                       \
     __global__ void __launch_bounds__(K2_THREADS, (EXACT) ? K2_MIN_CTAS_V1 : K2_MIN_CTAS)                                  \
-    NAME(DevIndex ix, DevParams p, DevBatch B, DevWork W0, size_t paths_stride, size_t hist_stride, size_t ckey_stride,     \
-         size_t cks_stride, size_t elist_stride, size_t order_stride, size_t rlist_stride, size_t clu_stride,              \
-         size_t dir_stride) {                                                                                              \
+    NAME(DevIndex ix, DevParams p, DevBatch B, DevWork W0, DevWorkStrides S) {                                             \
         extern __shared__ __align__(16) unsigned char smem_raw[];                                                          \
-        K2Shared *sh = (K2Shared *) smem_raw;                                                                              \
-        const size_t slot = blockIdx.x;                                                                                    \
-        DevWork W;                                                                                                         \
-        W.paths = W0.paths + slot * paths_stride;                                                                          \
-        W.hist = W0.hist + slot * hist_stride;                                                                             \
-        W.wlist = W0.wlist + slot * cks_stride;                                                                            \
-        W.ckey = W0.ckey + slot * ckey_stride;                                                                             \
-        W.cks = W0.cks + slot * cks_stride;                                                                                \
-        W.elist = W0.elist + slot * elist_stride;                                                                          \
-        W.order = W0.order + slot * order_stride;                                                                          \
-        W.rlist = W0.rlist + slot * rlist_stride;                                                                          \
-        W.clu = W0.clu + slot * clu_stride;                                                                                \
-        W.dir = W0.dir + slot * dir_stride;                                                                                \
-        W.max_blocks = W0.max_blocks;                                                                                      \
-        W.rl_cap = W0.rl_cap;                                                                                              \
-        unc_k2_cta_main<EXACT, FLAGS>(ix, p, B, W, sh);                                                                    \
+        unc_k2_cta_main<EXACT, FLAGS>(ix, p, B, unc_work_slot(W0, S, blockIdx.x), (K2Shared *) smem_raw);                 \
     }
 K2_MAP_KERNEL(k2_map, false, false)
 // ordered mode (unc_map_batch_ordered): per-read sources_added_ words in and out (kept out of k2_map, whose code is
@@ -217,7 +196,7 @@ struct unc_pool {
     unc_paf_rec *h_out = nullptr;  // pinned staging
     // workspaces
     DevWork W;
-    size_t paths_stride = 0, hist_stride = 0, ckey_stride = 0, cks_stride = 0, elist_stride = 0, order_stride = 0, rlist_stride = 0, clu_stride = 0, dir_stride = 0;
+    DevWorkStrides strides{};
     uint32_t n_slots = 0, grid = 0;
     size_t smem = 0;
     unc_timing last;
@@ -450,23 +429,25 @@ int unc_pool_create(const unc_index *idx, const unc_params *prm, uint32_t max_re
     // per-slot workspace sizes
     const size_t maxp = prm->max_paths;
     const size_t nchmax = (maxp + 31) / 32;
-    P->paths_stride = 2 * (nchmax * 160 + maxp) * 2;   // uint4: chunk-local child slots + sources, two generations
-    P->hist_stride = 24 * (nchmax * 160 + maxp);      // uint2: (C, parent) per record index, 24 generations
-    P->ckey_stride = 2 * maxp;        // uint4
-    P->cks_stride = nchmax * 160;     // uint4
-    P->elist_stride = nchmax * 32;    // uint4
-    P->order_stride = 2 * maxp;       // u32
-    if (const char *e = getenv("UNC_K2_SLOT_PAD")) {   // experiment knob: spread the slots over a larger address span
-        size_t f = (size_t) atoi(e);
-        if (f >= 2 && f <= 8) { P->paths_stride *= f; P->hist_stride *= f; P->ckey_stride *= f; P->cks_stride *= f; P->elist_stride *= f; P->order_stride *= f; }
-    }
+    DevWorkStrides &S = P->strides;
+    S.paths = 2 * (nchmax * 160 + maxp) * 2;   // uint4: chunk-local child slots + sources, two generations
+    S.hist = 24 * (nchmax * 160 + maxp);      // uint2: (C, parent) per record index, 24 generations
+    S.ckey = 2 * maxp;        // uint4
+    S.cks = nchmax * 160;     // uint4
+    S.elist = nchmax * 32;    // uint4
+    S.order = 2 * maxp;       // u32
     uint64_t longest = max_samples < 0xFFFFFFFFull ? max_samples : 0xFFFFFFFFull;
     // seed clusters: at most a few per event in practice; blocks are >= half full after splits
     uint64_t ev_cap = std::min<uint64_t>(prm->max_events, longest / 3 + 16);
     uint64_t mb = std::max<uint64_t>(1024, ev_cap * 2);
     mb = std::min<uint64_t>(mb, 1u << 17);
     const size_t rl_cap = 64 * 1024;   // seed rows of one event (typically tens)
-    size_t per_slot = (P->paths_stride + P->ckey_stride + 2 * P->cks_stride + P->elist_stride) * 16 + P->hist_stride * 8 + P->order_stride * 4 + 2 * rl_cap * 8 + mb * (UNC_BLK * 32 + 16);
+    S.rlist = 2 * rl_cap;
+    S.clu = (size_t) mb * UNC_BLK * 2;
+    S.dir = (size_t) mb + 1;
+    P->W.rl_cap = (u32) rl_cap;
+    P->W.max_blocks = (u32) mb;
+    size_t per_slot = (S.paths + S.ckey + 2 * S.cks + S.elist) * 16 + S.hist * 8 + S.order * 4 + S.rlist * 8 + S.clu * 16 + S.dir * 16;
     size_t free_b = 0, total_b = 0;
     PT(cudaMemGetInfo(&free_b, &total_b));
     size_t fixed = max_samples * 4 + (size_t) max_reads * (sizeof(DevReadDesc) + sizeof(DevRec) + 20) + (64u << 20);
@@ -476,22 +457,17 @@ int unc_pool_create(const unc_index *idx, const unc_params *prm, uint32_t max_re
     while ((size_t) grid * per_slot > budget && grid > 1) grid--;
     P->grid = grid;
     P->n_slots = grid;
-    P->rlist_stride = 2 * rl_cap;
-    P->W.rl_cap = (u32) rl_cap;
-    P->clu_stride = (size_t) mb * UNC_BLK * 2;
-    P->dir_stride = (size_t) mb + 1;
-    P->W.max_blocks = (u32) mb;
-    PT(cudaMalloc(&P->W.paths, (size_t) P->n_slots * P->paths_stride * 16));
-    PT(cudaMalloc(&P->W.ckey, (size_t) P->n_slots * P->ckey_stride * 16));
-    PT(cudaMalloc(&P->W.hist, (size_t) P->n_slots * P->hist_stride * 8));
-    PT(cudaMemset(P->W.hist, 0, (size_t) P->n_slots * P->hist_stride * 8));
-    PT(cudaMalloc(&P->W.wlist, (size_t) P->n_slots * P->cks_stride * 16));
-    PT(cudaMalloc(&P->W.cks, (size_t) P->n_slots * P->cks_stride * 16));
-    PT(cudaMalloc(&P->W.elist, (size_t) P->n_slots * P->elist_stride * 16));
-    PT(cudaMalloc(&P->W.order, (size_t) P->n_slots * P->order_stride * 4));
-    PT(cudaMalloc(&P->W.rlist, (size_t) P->n_slots * P->rlist_stride * 8));
-    PT(cudaMalloc(&P->W.clu, (size_t) P->n_slots * P->clu_stride * 16));
-    PT(cudaMalloc(&P->W.dir, (size_t) P->n_slots * P->dir_stride * 16));
+    PT(cudaMalloc(&P->W.paths, (size_t) P->n_slots * S.paths * 16));
+    PT(cudaMalloc(&P->W.ckey, (size_t) P->n_slots * S.ckey * 16));
+    PT(cudaMalloc(&P->W.hist, (size_t) P->n_slots * S.hist * 8));
+    PT(cudaMemset(P->W.hist, 0, (size_t) P->n_slots * S.hist * 8));
+    PT(cudaMalloc(&P->W.wlist, (size_t) P->n_slots * S.cks * 16));
+    PT(cudaMalloc(&P->W.cks, (size_t) P->n_slots * S.cks * 16));
+    PT(cudaMalloc(&P->W.elist, (size_t) P->n_slots * S.elist * 16));
+    PT(cudaMalloc(&P->W.order, (size_t) P->n_slots * S.order * 4));
+    PT(cudaMalloc(&P->W.rlist, (size_t) P->n_slots * S.rlist * 8));
+    PT(cudaMalloc(&P->W.clu, (size_t) P->n_slots * S.clu * 16));
+    PT(cudaMalloc(&P->W.dir, (size_t) P->n_slots * S.dir * 16));
     PT(cudaMalloc(&P->d_samples, max_samples * 4 + 64));
     PT(cudaMalloc(&P->d_reads, (size_t) max_reads * sizeof(DevReadDesc)));
     PT(cudaMallocHost(&P->h_reads, (size_t) max_reads * sizeof(DevReadDesc)));
@@ -636,17 +612,9 @@ static int batch_enqueue(unc_pool *P, const unc_read_desc *reads, uint32_t n, co
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaEventRecord(P->ev[2], s));
     uint32_t grid = std::min<uint32_t>(P->grid, n);
-    if (P->tie_order)
-        k2_map_exact<<<grid, K2_THREADS, P->smem, s>>>(P->idx->ix, P->dp, B, P->W, P->paths_stride, P->hist_stride, P->ckey_stride,
-                                                       P->cks_stride, P->elist_stride, P->order_stride, P->rlist_stride,
-                                                       P->clu_stride, P->dir_stride);
-    else if (h_flags_in)
-        k2_map_ord<<<grid, K2_THREADS, P->smem, s>>>(P->idx->ix, P->dp, B, P->W, P->paths_stride, P->hist_stride, P->ckey_stride,
-                                                     P->cks_stride, P->elist_stride, P->order_stride, P->rlist_stride,
-                                                     P->clu_stride, P->dir_stride);
-    else
-        k2_map<<<grid, K2_THREADS, P->smem, s>>>(P->idx->ix, P->dp, B, P->W, P->paths_stride, P->hist_stride, P->ckey_stride, P->cks_stride,
-                                                 P->elist_stride, P->order_stride, P->rlist_stride, P->clu_stride, P->dir_stride);
+    if (P->tie_order) k2_map_exact<<<grid, K2_THREADS, P->smem, s>>>(P->idx->ix, P->dp, B, P->W, P->strides);
+    else if (h_flags_in) k2_map_ord<<<grid, K2_THREADS, P->smem, s>>>(P->idx->ix, P->dp, B, P->W, P->strides);
+    else k2_map<<<grid, K2_THREADS, P->smem, s>>>(P->idx->ix, P->dp, B, P->W, P->strides);
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaEventRecord(P->ev[3], s));
     CUDA_TRY(cudaMemcpyAsync(P->h_out, P->d_out, (size_t) n * sizeof(DevRec), cudaMemcpyDeviceToHost, s));

@@ -1,6 +1,6 @@
 // unc_k2v2.cuh -- the mapper's worker warps, second structure (included by unc_device.cuh).
 //
-// Same results as unc_k2_workers (the first structure, kept for the exact-ties kernel): the reference's
+// Same results as unc_k2_workers_exact (the first structure, the exact-ties kernels' worker): the reference's
 // map_next (src/mapper.cpp:433-663) minus the seed clustering, which the tracker warp runs.  What changed
 // is how an event's work is laid out on the CTA:
 //
@@ -85,11 +85,7 @@ UNC_DEV bool k2v2_less_pre(u32 ax, u32 ay, u32 af, u32 ar, u32 bx, u32 by, u32 b
 // the bucket's span needs, then runs of equal fm_start ordered by (fm_end, seed_prob, record index).
 // `tmp` is the ping-pong partner of `keys` (same index range), `hist` 256 warp-private counters.
 // The sorted keys end in `keys`.
-#ifdef K2V2_SORT_NOINLINE
-UNC_DEV_NOINLINE
-#else
 UNC_DEV
-#endif
 void k2v2_sort_big(uint4 *keys, uint4 *tmp, u32 o, u32 n, u32 lo, u32 span_bits, u32 *hist) {
     const int lane = w_lane();
     const u32 lt = w_lanemask_lt();
